@@ -17,10 +17,15 @@ sharded `x.chunk(N)` across N GPUs; a "step" is ONE remote call (scatter → exe
 `--impl reference` times the reference's own CPU dispatch path on the host cores: the UNMODIFIED reference
 runtime from baseline/_ref (FastAPI app → supervisor → spawned ProcessWorkers, `kind: "reference"`) with
 N = --gpus ranks on a 64 MiB sample of the same workload; when baseline/_ref is absent, the oracle port.
+
+`--dump-outputs DIR` writes what the timed path returned in its last timed step: `DIR/result_sample.npy`, the
+results at a fixed, seeded sample of 4 Mi positions (float32, 16 MiB; the full result is 256 MiB).  The input is
+generated from a fixed seed, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -29,6 +34,10 @@ import sys
 import tempfile
 import threading
 import time
+
+# the tree may be read-only: no bytecode caches from this process or the rank processes it starts
+sys.dont_write_bytecode = True
+os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
 
 REPO = os.path.dirname(os.path.abspath(__file__))
 if REPO not in sys.path:
@@ -48,6 +57,24 @@ UNIT = "GB/s"
 REF_SAMPLE_ELEMS = 1 << 24   # 64 MiB arg per reference call (the reference needs seconds per call; 256 MiB exceeds its
                              # nginx body cap anyway, SURVEY.md §8(d))
 REF_DIR = os.path.join(REPO, "baseline", "_ref")
+INPUT_SEED = 0
+DUMP_SAMPLE = 1 << 22        # result positions written by --dump-outputs
+DUMP_SEED = 1234
+
+
+def timed_input():
+    """The timed call's argument: 64 Mi fp32 drawn on the host from a fixed seed (the same on every device and run)."""
+    import torch
+
+    return torch.randn(N_ELEMS, dtype=torch.float32, generator=torch.Generator().manual_seed(INPUT_SEED))
+
+
+def dump_index(device):
+    """The fixed, seeded sample of result positions --dump-outputs writes, sorted."""
+    import torch
+
+    idx = torch.randint(0, N_ELEMS, (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(DUMP_SEED))
+    return idx.sort().values.to(device)
 
 
 def workload_config(n_gpus: int) -> dict:
@@ -85,6 +112,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(
                 ["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "100", "-i",
                  str(self.index)], stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)   # the sampler never outlives the benchmark, even when a section fails
             self._t = threading.Thread(target=self._read, daemon=True)
             self._t.start()
         except Exception:  # noqa: BLE001
@@ -281,6 +309,7 @@ def _oracle_result(x, op, alpha, beta, world):
 def run_ours(args):
     import ctypes
 
+    import numpy as np
     import torch
     import torch.distributed as dist
 
@@ -316,10 +345,11 @@ def run_ours(args):
     # through the very same functions.
     TIMED = (N_ELEMS, 1, L.F32, L.OP_SCALE, 2.0, 0.0, 0)
     x = y = None
+    x_src = timed_input() if rank == 0 else None
     if world == 1:
         devices = list(range(n_gpus))
         ops.ensure_init(devices)
-        x = torch.randn(N_ELEMS, dtype=torch.float32, device="cuda:0")
+        x = x_src.to("cuda:0")
         y = torch.empty_like(x)
         x_ptr, y_ptr = x.data_ptr(), y.data_ptr()
         c_devs = L.arr(ctypes.c_int, devices)
@@ -354,7 +384,7 @@ def run_ours(args):
             ax, ay = ops.Arena(dev, nbytes), ops.Arena(dev, nbytes)
             mine["x"], mine["y"] = ax.export(), ay.export()
             x, y = ax.tensor(torch.float32), ay.tensor(torch.float32)
-            x.normal_()
+            x.copy_(x_src)
             torch.cuda.synchronize()
             x_ptr, y_ptr = ax.ptr, ay.ptr
         everyone = [None] * world
@@ -443,7 +473,7 @@ def run_ours(args):
                         raise SystemExit(f"PARITY FAILURE over real peers: case {name}, mode {mode}, N={n_gpus}")
                     report["cases"] += 1
         if rank == 0:   # restore the timed input
-            x.normal_()
+            x.copy_(x_src)
             torch.cuda.synchronize()
         sync_all()
         return report
@@ -470,11 +500,15 @@ def run_ours(args):
             ms = float(t.item())
         return ms / K, t0w, t1w
 
-    def check_result(tag):
+    last_outputs = {}   # mode -> the dump sample of what that mode's last timed call returned
+
+    def check_result(tag, mode):
         if rank == 0:
             idx = torch.randint(0, N_ELEMS, (4096,), device=x.device)
             assert torch.equal(y[idx], x[idx] * 2), f"{tag}: timed kernel produced wrong results"
             assert torch.equal(y[-1024:], x[-1024:] * 2), f"{tag}: tail wrong"
+            if args.dump_outputs:
+                last_outputs[mode] = y[dump_index(y.device)].cpu()
             y.zero_()
             torch.cuda.synchronize()
         if world > 1:
@@ -511,11 +545,11 @@ def run_ours(args):
         time.sleep(0.25)
     modes = {}
     ms_pull, t_wall0, t_wall1 = time_mode(call_pull)
-    check_result("pull")
+    check_result("pull", "pull_push_fused_kernel")
     modes["pull_push_fused_kernel"] = ms_pull
     if n_gpus > 1 and call_push is not None:
         ms_push, t0b, t_wall1 = time_mode(call_push)
-        check_result("push")
+        check_result("push", "push_push_flag_pipeline")
         modes["push_push_flag_pipeline"] = ms_push
     two_in_flight = None
     if world > 1:
@@ -525,7 +559,7 @@ def run_ours(args):
         # complete scatter -> exec -> gather whose results are checked below; nothing is skipped, calls only overlap.
         try:
             ms2 = time_two_in_flight()
-            check_result("push, two calls in flight")
+            check_result("push, two calls in flight", "push_push_flag_pipeline_two_calls_in_flight")
             modes["push_push_flag_pipeline_two_calls_in_flight"] = ms2
             two_in_flight = {"ms_per_step": ms2, "arg_plus_result_gbps": 2 * nbytes / (ms2 * 1e-3) / 1e9,
                              "root_port_gbps_per_direction": (n_gpus - 1) / n_gpus * nbytes / (ms2 * 1e-3) / 1e9,
@@ -537,6 +571,9 @@ def run_ours(args):
     # The timed region lasts a few milliseconds — shorter than one nvidia-smi sample — so the clocks are sampled over
     # an extended loop of the SAME call right after it (~0.6 s under load, all ranks take part).
     best_mode = min(modes, key=modes.get)
+    if rank == 0 and args.dump_outputs:   # the mode `value` reports
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "result_sample.npy"), last_outputs[best_mode].numpy())
     if best_mode == "pull_push_fused_kernel" or call_push is None:
         probe_fn = call_pull
     elif best_mode.endswith("two_calls_in_flight"):
@@ -1013,13 +1050,16 @@ def _traffic(n_gpus: int) -> dict:
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps (remote calls) of the headline measurement")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-c3", action="store_true")
     ap.add_argument("--push-chunks", type=int, default=32, help="chunks per shard of the push/push flag pipeline")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a sample of the last timed step's result to DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

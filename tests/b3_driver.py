@@ -1,12 +1,13 @@
-"""Child process of tests/test_b3_seam.py (authoring container only: needs /root/reference).
+"""Child process of oracle/make_b3_golden.py, which records tests/golden/b3_seam.json (needs the reference tree).
 
 Runs the UNMODIFIED reference server (kubetorch.serving.http_server:app under fastapi's TestClient, as the
 reference's own tests/test_http_server.py:86-96 does) with ONE change: the 3-line hook INTEGRATION.md gives for
 kubetorch/serving/supervisor_factory.py, applied by monkeypatching.  The server then builds B200Supervisor exactly
 as it builds its own supervisors — `supervisor_factory(**json.loads(KT_DISTRIBUTED_CONFIG))`, callable from the
 KT_* environment, RAW request bodies into SUPERVISOR.call — and the reference's CLIENT codecs
-(_serialize_body / _deserialize_response) sit on both ends.  The device layer is stubbed with torch CPU ops
-(`--stub`), because this container has no GPU; on a GPU box pass `--device` to run the real kernels."""
+(_serialize_body / _deserialize_response) sit on both ends.  Prints every exchange: the request body the reference
+client sent and the status and JSON body the reference server answered.  The device layer is stubbed with torch
+CPU ops (`--stub`, what tests/test_b3_seam.py replays against); pass `--device` to run the real kernels."""
 import json
 import os
 import sys
@@ -126,17 +127,16 @@ def main():
             ser = call.get("serialization", "pickle")
             body = _serialize_body(build_call_body(*args, **dict(call.get("kwargs") or {})), ser)
             url = f"/{cfg['callable']}" + (f"/{call['method']}" if call.get("method") else "")
+            request = json.loads(json.dumps(body))        # what goes on the wire (the server may consume `body`)
             resp = client.post(url, json=body, headers={"X-Serialization": ser, "X-Request-ID": "b3"})
-            rec = {"status_code": resp.status_code}
-            if resp.status_code == 200:
-                res = _deserialize_response(resp, ser)
-                rec["result"] = [{"dtype": str(t.dtype), "shape": list(t.shape), "data": t.reshape(-1).tolist()}
-                                 if isinstance(t, torch.Tensor) else t for t in res] if isinstance(res, list) else res
+            response = resp.json()
+            if resp.status_code != 200:
+                response.pop("traceback", None)           # host-specific file paths, not part of the contract
             else:
-                err = resp.json()
-                rec["error"] = {k: err.get(k) for k in ("error_type", "message", "pod_name", "detail") if k in err}
-            out.append(rec)
-    print("B3RESULT " + json.dumps({"records": out, "device_calls": stub.calls if stub else None}))
+                _deserialize_response(resp, ser)          # the reference client accepts the body
+            out.append({"path": url, "serialization": ser, "request": request, "status_code": resp.status_code,
+                        "response": response})
+    print("B3RESULT " + json.dumps({"exchanges": out, "device_calls": stub.calls if stub else None}))
 
 
 if __name__ == "__main__":      # the reference spawns workers for ITS supervisors; harmless here, kept for parity

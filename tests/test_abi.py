@@ -30,7 +30,9 @@ def test_library_exports_every_declared_symbol():
 def test_library_is_sm100a_only():
     import subprocess
 
-    out = subprocess.run(["cuobjdump", "-lelf", L.lib_path()], capture_output=True, text=True).stdout
+    from __graft_entry__ import cuda_tool
+
+    out = subprocess.run([cuda_tool("cuobjdump"), "-lelf", L.lib_path()], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_(\d+a?)", out))
     assert archs == {"100a"}, archs
 
@@ -41,7 +43,9 @@ def test_mlp_kernels_issue_tcgen05_and_tma_without_waterfall_loops():
     an ELECT + R2UR.BROADCAST + BRA.U.ANY loop (that form issued one MMA per ~177 cycles instead of 128)."""
     import subprocess
 
-    sass = subprocess.run(["cuobjdump", "-sass", L.lib_path()], capture_output=True, text=True).stdout
+    from __graft_entry__ import cuda_tool
+
+    sass = subprocess.run([cuda_tool("cuobjdump"), "-sass", L.lib_path()], capture_output=True, text=True).stdout
     funcs = sass.split("Function : ")[1:]
     wanted = {"gemm_bf16_tn_2sm_bres_kernel": 0, "gemm_bf16_tn_2sm_kernel": 0, "mlp_l2_head_fused_kernel": 0}
     for f in funcs:
